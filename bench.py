@@ -123,6 +123,27 @@ def make_inputs(W, H, D, need_right=False):
     return imL, vol
 
 
+DUMP_LIMIT_BYTES = 60 << 20   # data of all dumped arrays; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes what the timed path computed as out_dir/<name>.npy (float32), so that two builds can be compared output for output.
+    Arrays whose first axes are the image's H x W: when all of them together exceed DUMP_LIMIT_BYTES, the same seeded sample of
+    pixels (np.random.default_rng(0), ascending raster order) is taken from every one of them."""
+    os.makedirs(out_dir, exist_ok=True)
+    H, W = next(iter(arrays.values())).shape[:2]
+    total = sum(a.size * 4 for a in arrays.values())
+    idx = None
+    if total > DUMP_LIMIT_BYTES:
+        n = int(H * W * DUMP_LIMIT_BYTES // total)
+        idx = np.sort(np.random.default_rng(0).choice(H * W, n, replace=False))
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float32)
+        if idx is not None:
+            a = a.reshape((H * W,) + a.shape[2:])[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def all_planes(sweep, D):
     from localexpstereo_b200 import synth
     per_layer = [synth.synthetic_planes(sweep.layer(li).unitRegions, sweep.steps[li], D, 7 + li) for li in range(len(sweep.steps))]
@@ -384,7 +405,7 @@ def run_ours(args, W, H, D, windR, rank, world, local_rank):
             sweep_unary()
         run_u, graph_u = capture(sweep_unary)
         run_u(); run_u()
-        ms_u = timed(run_u, args.steps if naive else max(3, min(args.steps, 5)))
+        ms_u = timed(run_u, args.steps)
         unary_info = {"ms_per_step": ms_u, "value": evals_per_step / (ms_u * 1e-3), "unit": UNIT, "cuda_graph": graph_u,
                       "note": "the same 240 batched evaluations with host-supplied planes, unary maps written to an H x W image in HBM (no proposals, no update)"}
 
@@ -412,6 +433,9 @@ def run_ours(args, W, H, D, windR, rank, world, local_rank):
             clocks.start()
         ms_per_step = timed(run_pm, args.steps)
         clk = clocks.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:   # the state after the last timed step: currentCost_ / currentLabeling_
+            st_c, st_l = pms.get()
+            dump_outputs(args.dump_outputs, {"current_cost": st_c, "current_labeling": st_l})
         launches = launches_per_step * args.steps
         graph_used = graph_pm
         local_alg = unary.local_alg_bytes   # same cells, same K = 9/3/3 evaluations per cell visit as the unary sweep
@@ -420,6 +444,8 @@ def run_ours(args, W, H, D, windR, rank, world, local_rank):
             clocks.start()
         ms_per_step = timed(run_u, args.steps)
         clk = clocks.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:   # the unary maps of the last timed step, as written into the H x W cost image
+            dump_outputs(args.dump_outputs, {"cost_image": cost_d.cpu().numpy()})
         launches = unary.launches_per_sweep * args.steps
         graph_used = graph_u
         local_alg = unary.local_alg_bytes
@@ -456,7 +482,7 @@ def run_ours(args, W, H, D, windR, rank, world, local_rank):
         by_layer = {str(evs[i][0]): round(evs[i][1].elapsed_time(evs[i + 1][1]), 4) for i in range(len(evs) - 1)}
 
     # ---- end to end: the same sweep through the C-ABI with HOST buffers, copies inside the timed region
-    n_e2e = max(1, min(args.steps, 3))
+    n_e2e = args.steps
     e2e_unary = None
     if naive or world == 1:
         cost_h = np.zeros((H, W), np.float32)
@@ -472,10 +498,10 @@ def run_ours(args, W, H, D, windR, rank, world, local_rank):
         sweep_host()  # warm-up (allocates the pinned staging buffers)
         barrier()
         t0 = time.perf_counter()
-        for _ in range(1 if not naive else n_e2e):
+        for _ in range(n_e2e):
             sweep_host()
         torch.cuda.synchronize(dev)
-        dt = (time.perf_counter() - t0) / (1 if not naive else n_e2e)
+        dt = (time.perf_counter() - t0) / n_e2e
         L.host_unregister(cost_h)
         for ph in planes_h:
             L.host_unregister(ph)
@@ -547,7 +573,7 @@ def run_ours(args, W, H, D, windR, rank, world, local_rank):
             "config": {"workload": args.workload, "W": W, "H": H, "ndisp": D, "windR": windR, "th_col": TH_COL, "eps": EPS,
                        "layers_unit": unary.unit_sizes, "steps_per_layer": unary.steps,
                        "evals_per_step": evals_per_step, "target_px_per_step": unary.total_target_px,
-                       "batched_evaluations_per_step": launches // max(args.steps, 1),
+                       "batched_evaluations_per_step": launches // args.steps,
                        "parallelism": par, "cuda_graph": graph_used,
                        "l2": "inputs larger than L2 (cost volume %.2f GB; proposals follow the evolving state)" % (4.0 * D * H * W / 1e9)},
             "clocks": clk,
@@ -587,10 +613,15 @@ def main():
     ap.add_argument("--workload", default="synthetic_2048x1536x256_r20", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the sweep eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path computed in its last step to DIR/<name>.npy (float32, at most "
+                         "64 MB in all: a seeded sample of pixels beyond that); the inputs depend only on the arguments")
     ap.add_argument("--replicas", action="store_true",
                     help="BASELINE.json configs[3] style: every rank sweeps its OWN image pair (weak scaling, no data-path collective) "
                          "instead of sharding the cells of one pair (default, strong scaling)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     W, H, D, windR = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))

@@ -47,8 +47,11 @@ int fail(int code, const std::string& msg) {
 #define LEXP_CUDA(expr)                                                                                  \
     do {                                                                                                 \
         cudaError_t e__ = (expr);                                                                        \
-        if (e__ != cudaSuccess)                                                                          \
-            return fail(LEXP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e__));            \
+        if (e__ != cudaSuccess) {                                                                        \
+            std::string m__ = std::string(#expr) + ": " + cudaGetErrorString(e__);                      \
+            cudaGetLastError(); /* reset: a launch check after this failure must not report it again */  \
+            return fail(LEXP_ERR_CUDA, m__);                                                             \
+        }                                                                                                \
     } while (0)
 
 // futex on a 32-bit word: block while *addr == expected / wake every waiter (the combiner's followers sleep in the kernel instead of
@@ -342,6 +345,18 @@ void* mapped_alias(void* p, size_t bytes) {
             static_cast<char*>(a1.devicePointer) - static_cast<char*>(a0.devicePointer) != (ptrdiff_t)(bytes - 1)) { cudaGetLastError(); return nullptr; }
     }
     return a0.devicePointer;
+#endif
+}
+
+// p lies in page-locked host memory that CUDA knows of (cudaHostRegister / cudaHostAlloc)
+bool registered_host(const void* p) {
+#ifdef LEXP_EMU
+    void* d = nullptr;
+    return cudaHostGetDevicePointer(&d, const_cast<void*>(p), 0) == cudaSuccess && d;
+#else
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    return a.type == cudaMemoryTypeHost;
 #endif
 }
 
@@ -902,6 +917,12 @@ int lexp_plan_eval_host_tiles(lexp_ctx* c, lexp_plan* pl, int mode, const lexp_p
     { int rc0 = ensure_compact(pl, nout); if (rc0) return rc0; }
     int rc = run_plan(c, pl, mode, pl->d_planes, pl->d_compact, 0, 1, with_check);
     if (rc) return rc;
+    if (registered_host(tiles)) {  // starts inside a registration that does not cover it: one copy cannot span both kinds of memory
+        LEXP_CUDA(cudaMemcpyAsync(pl->h_compact, pl->d_compact, nout * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        LEXP_CUDA(cudaStreamSynchronize(c->stream));
+        memcpy(tiles, pl->h_compact, nout * sizeof(float));
+        return LEXP_OK;
+    }
     LEXP_CUDA(cudaMemcpyAsync(tiles, pl->d_compact, nout * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     LEXP_CUDA(cudaStreamSynchronize(c->stream));
     return LEXP_OK;

@@ -267,5 +267,10 @@ def test_bench_cpu_baseline_block_of_the_gpu_arm():
     cpu = bench.cpu_baseline_beside(W, H, D, windR, imL, vol, False, None, groups, lambda l: layers[l], planes)
     assert cpu["value"] > 0 and cpu["kind"] in ("reference", "port") and cpu["cores"] >= 1 and "L0g0x3+L1g0x2" in cpu["sample"]
     imR = synth.synthetic_image(H, W, 43)
+    from oracle import build_ref
+    if build_ref.build() is None:   # the image-based energy's only CPU implementation is the compiled reference
+        with pytest.raises(RuntimeError, match="no CPU implementation"):
+            bench.cpu_baseline_beside(W, H, D, windR, imL, None, True, imR, groups, lambda l: layers[l], planes)
+        return
     cpu = bench.cpu_baseline_beside(W, H, D, windR, imL, None, True, imR, groups, lambda l: layers[l], planes)
     assert cpu["value"] > 0 and cpu["kind"] == "reference"
