@@ -166,8 +166,7 @@ LEXP_API int lexp_set_overlap(lexp_ctx* ctx, int on);
 LEXP_API int64_t lexp_launch_count(const lexp_ctx* ctx);
 /* Concurrent lexp_eval_cell calls (the OpenMP loop of FastGCStereo.h:30-49, one blocking call per cell and thread) are
  * combined: calls that arrive while the device is busy are evaluated together in one batched launch.  Returns how many
- * such launches there were and how many calls they served (calls that found the device idle are not counted).
- * LEXP_COMBINE=0 in the environment at lexp_create disables the combining. */
+ * such launches there were and how many calls they served (calls that found the device idle are not counted). */
 LEXP_API int lexp_combine_stats(const lexp_ctx* ctx, int64_t* batches, int64_t* calls);
 
 /* ---- PatchMatch phase on the device: FastGCStereo::run's `pmInit` iterations (FastGCStereo.h:143-157), i.e.

@@ -12,7 +12,7 @@ DEPS = SRCS + [os.path.join(HERE, "csrc", "lexp_kernels.cuh"), os.path.join(HERE
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
-    "-Xcompiler", "-fPIC,-fvisibility=hidden", "-shared", "--use_fast_math=false" if False else "-Xptxas=-v",
+    "-Xcompiler", "-fPIC,-fvisibility=hidden", "-shared", "-Xptxas=-v",
 ]
 
 
@@ -24,7 +24,7 @@ def needs_build():
 
 
 def build(force=False, verbose=False):
-    # LEXP_NVCC_DEFS: extra -D flags for build-time kernel variants (experiments only, e.g. "-DLEXP_STATS_TMA=1"); a variant build is
+    # LEXP_NVCC_DEFS: extra -D flags for build-time kernel variants (diagnosis only, e.g. "-DLEXP_TRACE=1"); a variant build is
     # always forced and the next plain build() restores the default kernel because the .so is older than this marker
     extra = os.environ.get("LEXP_NVCC_DEFS", "").split()
     marker = SO + ".variant"

@@ -140,16 +140,12 @@ struct lexp_ctx {
     int tile_oh = 128;    // max output rows per work item
     bool tile_oh_fixed = false;  // LEXP_TILE_OH given: no per-plan search
     int num_sms = 148;
-    int ctas_per_sm = kMinCtas;  // CTA slots per SM the planner fills (LEXP_CTAS_PER_SM)
-    bool pdl = false;            // launch with programmatic stream serialization (builds with -DLEXP_PDL=1; LEXP_PDL_OFF=1 disables)
     bool overlap = false;        // lexp_set_overlap: launches with device-resident planes may overlap their predecessors
     bool chain_ok = false;       // the last operation this context put on its stream was a launch of lexp_fused_kernel: only then may the
                                  // next launch carry the programmatic-serialization attribute.  After a memcpy / memset (plane upload, counter
                                  // reset, state upload) the next launch is an ordinary one: a kernel launched with the attribute right after a
                                  // copy was observed reading the copy's destination before the copy had landed
-    size_t smem_cap = 0;         // upper bound on a work item's dynamic shared memory, 0: none (LEXP_SMEM_CAP)
     size_t smem_limit = 0;
-    size_t window_max = 0;
     bool smem_configured[2] = {false, false};
     bool own_stream = true;
     bool vol_finite[2] = {false, false};
@@ -185,7 +181,6 @@ struct lexp_ctx {
     std::atomic<int> comb_n{0};    // = comb_q.size(), readable without the mutex (the leader's collection window polls it)
     std::atomic<int> comb_gen{0};  // bumped (and futex-woken) whenever requests change state: what waiting callers sleep on
     bool comb_leader = false;      // a leader is collecting / running a batch
-    bool combine = true;           // LEXP_COMBINE=0: every call on its own (the round-1 behaviour)
     int comb_window_us = 30;       // LEXP_COMBINE_WINDOW_US: how long a leader waits for the queue to stop growing
     std::atomic<size_t> comb_seen{1};   // largest batch so far: a leader stops collecting as soon as that many calls are queued
     struct CombBuf {               // staging of one batch: pinned (mapped) host memory, plus device copies of items / planes
@@ -255,8 +250,8 @@ int launch_fused_t(lexp_ctx* c, const KParams& kp_in, int nitems, size_t smem, b
         LEXP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_limit));
         c->smem_configured[PM] = true;
     }
-#if LEXP_PDL && !defined(LEXP_EMU)
-    if (c->pdl && allow_pdl && c->chain_ok) {  // programmatic dependent launch: see LEXP_PDL in lexp_kernels.cuh
+#ifndef LEXP_EMU
+    if (allow_pdl && c->chain_ok) {  // programmatic dependent launch: see lexp_kernels.cuh
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)nitems); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = c->stream;
         cudaLaunchAttribute at[1];
@@ -393,11 +388,10 @@ int run_plan(lexp_ctx* c, lexp_plan* pl, int mode, const Plane4* d_planes, float
         // (the cost-volume gathers are plain read-only loads; see profiles/r1_experiments.md)
         cudaStreamAttrValue av{};
         av.accessPolicyWindow.base_ptr = c->d_gs[mode];
-        // default: pin a prefix [statA | statC | guide | ..] of exactly the set-aside size with hit ratio 1 (measured 1 %
-        // better than LEXP_L2_PERSIST=2: the whole allocation with a fractional hit ratio)
-        const bool prefix = env_int("LEXP_L2_PERSIST", 1) != 2;
-        av.accessPolicyWindow.num_bytes = prefix ? std::min(c->gs_bytes, c->persist_bytes) : std::min(c->gs_bytes, c->window_max);
-        av.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)c->persist_bytes / (double)av.accessPolicyWindow.num_bytes);
+        // pin a prefix [statA | statC | guide | ..] of exactly the set-aside size with hit ratio 1 (measured 1 % better than a
+        // window over the whole allocation with a fractional hit ratio)
+        av.accessPolicyWindow.num_bytes = std::min(c->gs_bytes, c->persist_bytes);
+        av.accessPolicyWindow.hitRatio = 1.0f;
         av.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
         av.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
         if (cudaStreamSetAttribute(c->stream, cudaStreamAttributeAccessPolicyWindow, &av) == cudaSuccess) c->persist_mode = mode;
@@ -514,22 +508,15 @@ int lexp_create(const lexp_params* params, lexp_ctx** out_ctx) {
     c->tile_oh = std::max(8, env_int("LEXP_TILE_OH", 128));
     c->tile_oh_fixed = getenv("LEXP_TILE_OH") != nullptr;
     c->num_sms = prop.multiProcessorCount;
-    // kMinCtas CTAs must fit next to each other: 1 KB of every CTA's shared memory is reserved by the system.  With the
-    // default build (2 CTAs) no cap is needed: the widest tile needs ~93 KB.
-    c->ctas_per_sm = env_int("LEXP_CTAS_PER_SM", kMinCtas);
-    c->pdl = LEXP_PDL && !env_int("LEXP_PDL_OFF", 0);
-    c->combine = env_int("LEXP_COMBINE", 1) != 0;
     c->comb_window_us = std::max(0, env_int("LEXP_COMBINE_WINDOW_US", 30));
-    c->smem_cap = (size_t)env_int("LEXP_SMEM_CAP", 0);
     c->gc_threads = std::min(1024, std::max(32, env_int("LEXP_GC_THREADS", 1024) / 32 * 32));
     c->gc_relabel_every = std::max(1, env_int("LEXP_GC_RELABEL_EVERY", 24));
     c->gc_big_nodes = std::max(0, env_int("LEXP_GC_BIG_NODES", 32768));
+    // LEXP_L2_PERSIST=0 leaves the device-wide persisting-L2 limit untouched (other processes on a shared GPU see that limit)
     if (env_int("LEXP_L2_PERSIST", 1) && prop.persistingL2CacheMaxSize > 0) {
         const size_t want = (size_t)prop.persistingL2CacheMaxSize;
-        if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
-            c->persist_bytes = want;
-            c->window_max = (size_t)prop.accessPolicyMaxWindowSize;
-        } else cudaGetLastError();
+        if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) c->persist_bytes = want;
+        else cudaGetLastError();
         if (env_int("LEXP_DEBUG", 0))
             fprintf(stderr, "[lexp] L2 %d B, persisting max %d B, window max %d B, set-aside %zu B\n", prop.l2CacheSize,
                     prop.persistingL2CacheMaxSize, prop.accessPolicyMaxWindowSize, c->persist_bytes);
@@ -755,14 +742,12 @@ int lexp_plan_create(lexp_ctx* c, int n, const lexp_rect* filt, const lexp_rect*
     std::lock_guard<std::mutex> lk(c->mu);
     LEXP_CUDA(cudaSetDevice(c->p.device));
     const int R = c->R;
-    int ow_max = max_tile_ow(R);
-    if (c->smem_cap)  // narrower tiles so that every work item fits the per-CTA shared-memory budget of the build
-        while (ow_max > 8 && fused_smem_bytes(ow_max + 4 * R, 128, R) > c->smem_cap) ow_max -= 4;
-    // Row segmentation: every segment re-streams 4R warm-up rows, but more items fill the 2 x #SM CTA slots better.
+    const int ow_max = max_tile_ow(R);
+    // Row segmentation: every segment re-streams 4R warm-up rows, but more items fill the kMinCtas x #SM CTA slots better.
     // Pick the segment height that minimises  waves x (rows streamed per item)  for this plan.
     int oh_max = c->tile_oh;
     if (!c->tile_oh_fixed) {
-        const int64_t slots = (int64_t)c->ctas_per_sm * c->num_sms;
+        const int64_t slots = (int64_t)kMinCtas * c->num_sms;
         double best = 1e300;
         for (int cand = 24; cand <= 128; cand += 4) {
             int64_t items = 0;
@@ -1095,7 +1080,7 @@ int lexp_eval_cell(lexp_ctx* c, int mode, const lexp_rect* filt, const lexp_rect
             return rc2;
         }
     }
-    if (!c->combine || mode < 0 || mode > 1) return lexp_plan_eval_host(c, pl, mode, plane, base, step_bytes, with_check);
+    if (mode < 0 || mode > 1) return lexp_plan_eval_host(c, pl, mode, plane, base, step_bytes, with_check);
 
     lexp_ctx::CellReq req;
     req.mode = mode; req.with_check = with_check; req.pl = pl; req.plane = *plane; req.base = base; req.step_bytes = step_bytes;

@@ -28,55 +28,31 @@
 
 namespace lexp {
 
-#if defined(LEXP_STATS_TMA) && LEXP_STATS_TMA && !defined(LEXP_EMU)
-#define LEXP_TMA_ON 1
-#else
-#define LEXP_TMA_ON 0
-#endif
 constexpr int kWarpsA = 4, kWarpsH = 2, kWarpsC = 3, kWarpsE = 2;
-constexpr int kWarpsT = LEXP_TMA_ON;   // LEXP_STATS_TMA: a 12th warp whose lane 0 feeds team C's statistics ring through the TMA unit
-constexpr int kThreads = 32 * (kWarpsA + kWarpsH + kWarpsC + kWarpsE + kWarpsT);  // 352 (384)
+constexpr int kThreads = 32 * (kWarpsA + kWarpsH + kWarpsC + kWarpsE);  // 352
 constexpr int kMaxVW = 32 * kWarpsA;   // virtual tile width  ow + 4R
 constexpr int kMaxW2 = 32 * kWarpsC;   // (a,b) columns       ow + 2R
 constexpr int kMaxOW = 32 * kWarpsE;   // output columns
 constexpr int kRun = 8;                // columns per H task
 constexpr int kCH = 2;                 // rows per pipeline chunk
-// ---- build-time switches -------------------------------------------------------------------------------------------------
-// (round 2 measured and removed the three-CTAs-per-SM register diet and its ingredients -- rolling statistics prefetch, H re-reads,
-//  per-link buffer strides, 4-row gather batches: profiles/r2_variants.md)
-// LEXP_A_ROWTAB: the byte offset of a volume row inside the blocked layout, (y / 4) * block-row pitch + (y % 4) * 16, is looked up
+// ---- measured design choices (B200, profiles/r2_variants.md) ---------------------------------------------------------------
+// Row table: the byte offset of a volume row inside the blocked layout, (y / 4) * block-row pitch + (y % 4) * 16, is looked up
 //   in a per-tile shared-memory table (16-byte units, filled in the prologue next to the plane's b*y + c) instead of being
-//   recomputed with 64-bit multiplies for every row of every column: ~19 -> ~5 address instructions per gathered row in team A.
-// Measured on B200 (profiles/r2_variants.md): 17.56 -> 17.26 ms per sweep; default since round 2.
-#ifndef LEXP_A_ROWTAB
-#define LEXP_A_ROWTAB 1
-#endif
-// LEXP_PDL: programmatic dependent launch.  Every thread signals `griddepcontrol.launch_dependents` at the top of the kernel, so
-//   the NEXT batched evaluation of the stream (launched with the programmatic-stream-serialization attribute, lexp_capi.cu) may
+//   recomputed with 64-bit multiplies for every row of every column: ~19 -> ~5 address instructions per gathered row in team A,
+//   17.56 -> 17.26 ms per sweep.
+// Programmatic dependent launch (PDL): every thread signals `griddepcontrol.launch_dependents` at the top of the kernel, so the
+//   NEXT batched evaluation of the stream (launched with the programmatic-stream-serialization attribute, lexp_capi.cu) may
 //   occupy CTA slots as soon as all CTAs of this one are resident: it fills the partly empty last wave and hides the launch gap
 //   and its own prologue + 4R warm-up rows.  Consecutive launches write overlapping parts of the same cost image (the steps of a
 //   group), so team E executes `griddepcontrol.wait` (previous grids complete, their writes visible) before its first store;
-//   nothing else written by a previous launch is read.  Measured on B200 (profiles/r2_variants.md): 17.56 -> 15.49 ms per
-//   sweep (the 240 launches of a sweep replayed as one CUDA graph); default since round 2.  LEXP_PDL_OFF=1 disables it at run time.
-#ifndef LEXP_PDL
-#define LEXP_PDL 1
-#endif
+//   nothing else written by a previous launch is read.  17.56 -> 15.49 ms per sweep (the 240 launches of a sweep replayed as one
+//   CUDA graph).
+// ---- build-time switch -----------------------------------------------------------------------------------------------------
 // LEXP_TRACE: diagnosis build.  Every warp accumulates the clock cycles it spends waiting for its input link (consume_begin) and
 //   for a free output buffer (produce_begin) and writes {total, wait_in, wait_out, chunks} at the end; lexp_capi.cu averages
 //   them per team after every launch (LEXP_TRACE_FILE).  Shows directly which team the pipeline waits for.  Not a product build.
 #ifndef LEXP_TRACE
 #define LEXP_TRACE 0
-#endif
-// LEXP_STATS_TMA: team C's guided-filter statistics (36 of the 47 algorithmic bytes per eval: dense rectangular rows) are staged
-//   into a shared-memory ring by the TMA unit -- cp.async.bulk global -> shared, completion on an mbarrier -- LEXP_STATS_STAGES
-//   chunks ahead instead of being loaded into registers one chunk ahead.  ncu (profiles/r2_fused_ncu_L0.md): team C is the team
-//   the pipeline waits for and 29 % of its stall samples are long_scoreboard on exactly these loads; one chunk of lead (~1700
-//   cycles) does not cover a loaded DRAM round trip, a second register set spills (80-register cap), the ring costs no registers.
-#ifndef LEXP_STATS_TMA
-#define LEXP_STATS_TMA 0
-#endif
-#ifndef LEXP_STATS_STAGES
-#define LEXP_STATS_STAGES 4
 #endif
 constexpr int kMinCtas = 2;           // resident CTAs per SM the kernel is compiled for (register cap 65536 / (kMinCtas * kThreads))
 constexpr int kG = 6;                 // rows per gather batch of team A (one batch of loads in flight)
@@ -178,22 +154,11 @@ __host__ __device__ inline int srow_stride(int vw) {
     int s = sidx(vw + kRun + 7) + 1;
     return s + ((12 - (s & 7)) & 7);  // == 4 (mod 8) float4 units: the 2 rows x 4 runs of a quarter-warp hit 8 bank groups
 }
-// LEXP_STATS_TMA: one ring stage = one chunk of team C's statistics: statA / statB rows [kCH][w2] float4, statC rows [kCH][w2c] float
-// (w2c: room for the 16-byte alignment shift of a row start); then one mbarrier per stage
-__host__ __device__ inline int stats_w2c(int w2) { return (w2 + 7 + 3) & ~3; }
-__host__ __device__ inline int stats_stage_bytes(int w2) { return kCH * (2 * w2 * 16 + stats_w2c(w2) * 4); }
-__host__ __device__ inline size_t stats_ring_bytes(int w2) {
-#if LEXP_TMA_ON
-    return (size_t)LEXP_STATS_STAGES * stats_stage_bytes(w2) + 16 * LEXP_STATS_STAGES;   // stages, then a full and an empty mbarrier each
-#else
-    return 0;
-#endif
-}
 __host__ __device__ inline size_t fused_smem_bytes(int vw, int oh, int R) {
     const int K = 2 * R + 1;
     const int vh = oh + 4 * R;
     const int rows = 8 * kCH * srow_stride(vw);
-    return (size_t)((K * vw + 1) / 2 + K * (vw - 2 * R) + rows + 3 * ((vh + 3) / 4) + 3) * 16 + stats_ring_bytes(vw - 2 * R) + 16;  // + 6 doubles (NAIVE: inverse affine map) + statistics ring + the plane slot (PatchMatch phase) at the very end
+    return (size_t)((K * vw + 1) / 2 + K * (vw - 2 * R) + rows + 3 * ((vh + 3) / 4) + 3) * 16 + 16;  // + 6 doubles (NAIVE: inverse affine map) + the plane slot (PatchMatch phase) at the very end
 }
 
 // ---- packed f32x2 helpers (sm_100: FADD2 / FFMA2) --------------------------------------------
@@ -223,27 +188,6 @@ inline u64 sub2(u64 a, u64 b) { float a0, a1, b0, b1; up2(a, a0, a1); up2(b, b0,
 __device__ __forceinline__ F4 f4add(F4 a, F4 b) { return F4{add2(a.lo, b.lo), add2(a.hi, b.hi)}; }
 __device__ __forceinline__ F4 f4sub(F4 a, F4 b) { return F4{sub2(a.lo, b.lo), sub2(a.hi, b.hi)}; }
 __device__ __forceinline__ F4 f4zero() { return F4{0ull, 0ull}; }
-
-// ---- mbarrier + bulk asynchronous copy (TMA unit, non-tensor form: contiguous bytes global -> shared) ---------------------
-#if LEXP_TMA_ON
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory"); }
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-    unsigned ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-#endif
 
 // ---- named barriers: pairwise producer/consumer hand-off between warp teams ------------------------
 // link L (0: A->H1 via hb1, 1: H1->C via ho1, 2: C->H2 via hb2, 3: H2->E via ho2), buffer parity b:
@@ -435,7 +379,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
     LEXP_DYNAMIC_SMEM(smem_raw);
     F4* smem = reinterpret_cast<F4*>(smem_raw);
 
-#if LEXP_PDL && !defined(LEXP_EMU)
+#ifndef LEXP_EMU
     asm volatile("griddepcontrol.launch_dependents;");
 #endif
 #if LEXP_TRACE
@@ -471,47 +415,6 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
     float* s_dbase = s_invny + 4 * ((it.oh + 4 * R + 3) / 4);        // [VHs] b*y + c of the plane  (NAIVE: int X0 of the warp)
     int* s_Y0 = reinterpret_cast<int*>(s_dbase + 4 * ((it.oh + 4 * R + 3) / 4));  // [VHs] NAIVE: fixed-point source row
     double* s_iM = reinterpret_cast<double*>(s_Y0 + 4 * ((it.oh + 4 * R + 3) / 4));  // [6] NAIVE: inverse affine map of the call
-#if LEXP_TMA_ON
-    // statistics ring of team C (TMA unit): LEXP_STATS_STAGES stages, then their mbarriers; behind s_iM (6 doubles)
-    unsigned char* s_ring = reinterpret_cast<unsigned char*>(s_iM) + 48;
-    const int stageB = stats_stage_bytes(W2);
-    uint64_t* s_full = reinterpret_cast<uint64_t*>(s_ring + LEXP_STATS_STAGES * stageB);   // [NS] completed by the copies' bytes
-    uint64_t* s_empty = s_full + LEXP_STATS_STAGES;                                          // [NS] completed by team C's 96 threads
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < LEXP_STATS_STAGES; i++) { mbar_init(s_full + i, 1); mbar_init(s_empty + i, 32 * kWarpsC); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    const int st_xa = max(X0 + R, it.fx), st_xb = min(X0 + R + W2, fx1);   // columns of the tile's (a, b) strip inside the filterRect
-    // one chunk of statistics rows -> ring stage chunk % NS: up to 3 bulk copies per row (statA, statB: float4 rows; statC: a float row
-    // that starts at any float, copied from the 16-byte boundary below it), completion counted in bytes on the stage's mbarrier
-    auto tma_issue = [&](int chunk) {
-        unsigned char* stg = s_ring + (chunk % LEXP_STATS_STAGES) * stageB;
-        uint64_t* bar = s_full + (chunk % LEXP_STATS_STAGES);
-        const int W2c = stats_w2c(W2);
-        unsigned bytes = 0;
-#pragma unroll
-        for (int r = 0; r < kCH; r++) {
-            const int v = chunk * kCH + r;
-            if (v >= vC0 && v < vC1 && st_xb > st_xa)
-                bytes += 2u * (unsigned)(st_xb - st_xa) * 16u + (unsigned)(((((ys + v - R) * P.W + st_xa) & 3) + (st_xb - st_xa) + 3) & ~3) * 4u;
-        }
-        if (!bytes) { mbar_arrive(bar); return; }
-        mbar_expect_tx(bar, bytes);
-#pragma unroll
-        for (int r = 0; r < kCH; r++) {
-            const int v = chunk * kCH + r;
-            if (v >= vC0 && v < vC1 && st_xb > st_xa) {
-                const size_t g0 = (size_t)(ys + v - R) * P.W + st_xa;
-                const size_t so = (size_t)(r * W2 + (st_xa - (X0 + R))) * 16;
-                bulk_g2s(stg + so, P.statA + g0, (unsigned)(st_xb - st_xa) * 16u, bar);
-                bulk_g2s(stg + (size_t)kCH * W2 * 16 + so, P.statB + g0, (unsigned)(st_xb - st_xa) * 16u, bar);
-                const size_t g0a = g0 & ~(size_t)3;
-                bulk_g2s(stg + (size_t)2 * kCH * W2 * 16 + (size_t)r * W2c * 4, P.statC + g0a, (unsigned)(((int)(g0 - g0a) + (st_xb - st_xa) + 3) & ~3) * 4u, bar);
-            }
-        }
-    };
-#endif
 
     if (PM) {
         // PatchMatch phase.  (0) Group boundary: the previous group (this rank's and, on the multi-GPU cell shard, the peers') must
@@ -593,10 +496,8 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
             s_invny[v] = 1.0f / (float)(min(y + R, fy1 - 1) - max(y - R, it.fy) + 1);  // GuidedFilter.h:324
             if (!NAIVE) {
                 s_dbase[v] = __fadd_rn(__fmul_rn(pl.b, (float)y), pl.c);               // CostVolumeEnergy.h:73
-#if LEXP_A_ROWTAB
                 // row offset in the blocked volume, in 16-byte units (the s_Y0 slot is unused by the cost-volume energy)
                 reinterpret_cast<unsigned*>(s_Y0)[v] = (unsigned)(y >> 2) * ((unsigned)P.Wb * (unsigned)P.D * 4u) + (unsigned)(y & 3);
-#endif
             } else {
                 // cv::warpAffine fixed-point row terms (AB_BITS = 10, round_delta = 16) for the inverse affine map of
                 // StereoEnergy.h:704-729
@@ -695,13 +596,9 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
         const int XAc = colA ? XA : it.fx;
         // blocked volume: element (d, y, x) lives at ((((y/4) * Wb + x/4) * D + d) * 4 + y%4) * 4 + x%4:
         // a 128-byte line holds 2 disparities of a 4x4 pixel block, so the rows of a gather batch share lines
-#if !LEXP_A_ROWTAB
-        const size_t vblk = (size_t)P.Wb * P.D * 64;       // bytes per block row (4 image rows)
-#endif
         const char* vcol = reinterpret_cast<const char*>(P.vol) + ((size_t)(XAc >> 2) * P.D * 16 + (XAc & 3)) * 4;
-#if LEXP_A_ROWTAB && !defined(LEXP_EMU)
-        // keep the column base as ONE 64-bit pointer (otherwise: offset + uniform base, re-added per row); not with the 56-register
-        // diet, where the extra live register pair spills
+#ifndef LEXP_EMU
+        // keep the column base as ONE 64-bit pointer (otherwise: offset + uniform base, re-added per row)
         asm volatile("" : "+l"(vcol));
 #endif
         const char* grow = reinterpret_cast<const char*>(P.guide) + ((size_t)ys * P.W + XAc) * 4;
@@ -744,7 +641,6 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
                 lv0[j] = 0.f; lv1[j] = 0.f; lg[j] = 0u; lf1[j] = fast ? 0.f : -1.f;  // outside filterRect: zero
                 if (colA && vi < vReal) {
                     int d0, d1;
-#if LEXP_A_ROWTAB
                     const char* vrow = vcol + (size_t)reinterpret_cast<const unsigned*>(s_Y0)[vi] * 16;
                     if (fast) {  // the second sample is always the next disparity: 64 bytes further in the blocked layout
                         lf1[j] = weights(__fadd_rn(ax, s_dbase[vi]), d0, d1);  // :76
@@ -757,13 +653,6 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
                         lv0[j] = ldg_stream(p0);
                         lv1[j] = ldg_stream(p0 + ((d1 - d0) << 4));  // d1 - d0 is 1, or 0 when the sampler clamps at D - 1
                     }
-#else
-                    lf1[j] = weights(__fadd_rn(ax, s_dbase[vi]), d0, d1);  // :76
-                    const int y = ys + vi;
-                    const char* vrow = vcol + (size_t)(y >> 2) * vblk + (y & 3) * 16;
-                    lv0[j] = ldg_stream(reinterpret_cast<const float*>(vrow + (size_t)(unsigned)d0 * 64));
-                    lv1[j] = ldg_stream(reinterpret_cast<const float*>(vrow + (size_t)(unsigned)d1 * 64));
-#endif
                     lg[j] = __ldg(reinterpret_cast<const unsigned int*>(grow));
                 }
                 vi++;
@@ -899,37 +788,17 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
         const float4* pb = P.statB + pix0;
         const float* pc = P.statC + pix0;
         auto issue = [&]() {
-#if LEXP_TMA_ON
-            if (vi < nChunks * kCH) mbar_wait(s_full + ((vi / kCH) % LEXP_STATS_STAGES), (unsigned)(((vi / kCH) / LEXP_STATS_STAGES) & 1));
-#endif
 #pragma unroll
             for (int r = 0; r < kCH; r++) {
                 sa[r] = make_float4(0.f, 0.f, 0.f, 0.f); sb[r] = sa[r]; sc[r] = 0.f;
-#ifdef LEXP_X_NOSTATS
-                if (colC && vi >= vC0 && vi < vC1) { sa[r] = make_float4(0.5f, 0.5f, 0.5f, 10.f); sb[r] = make_float4(0.f, 0.f, 10.f, 0.f); sc[r] = 10.f; }
-                if (false) {
-#else
                 if (colC && vi >= vC0 && vi < vC1) {
-#endif
-#if LEXP_TMA_ON
-                    // the row was staged by the TMA unit (team H2 issues the copies LEXP_STATS_STAGES chunks ahead): shared-memory reads,
-                    // one chunk ahead of their use like the global loads they replace
-                    const unsigned char* stg = s_ring + ((vi / kCH) % LEXP_STATS_STAGES) * stageB;
-                    sa[r] = reinterpret_cast<const float4*>(stg)[r * W2 + t];
-                    sb[r] = reinterpret_cast<const float4*>(stg + (size_t)kCH * W2 * 16)[r * W2 + t];
-                    sc[r] = reinterpret_cast<const float*>(stg + (size_t)2 * kCH * W2 * 16)[r * stats_w2c(W2) + (((ys + vi - R) * P.W + st_xa) & 3) + (XC - st_xa)];
-#else
                     sa[r] = __ldg(pa);
                     sb[r] = __ldg(pb);
                     sc[r] = __ldg(pc);
-#endif
                 }
                 vi++;
                 pa += P.W; pb += P.W; pc += P.W;
             }
-#if LEXP_TMA_ON
-            if (vi <= nChunks * kCH) mbar_arrive(s_empty + ((vi / kCH - 1) % LEXP_STATS_STAGES));   // this thread has read the stage
-#endif
         };
         issue();
         for (int c = 0; c < nChunks; c++) {
@@ -1016,14 +885,10 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
 #pragma unroll
             for (int r = 0; r < kCH; r++) {
                 gq[r] = 0u; cq[r] = 0.f;
-#ifdef LEXP_X_NOGUIDE_E
-                if (colE && vi >= vE0 && vi < VHs) gq[r] = 0x00808080u;
-#else
                 if (colE && vi >= vE0 && vi < VHs) {
                     gq[r] = __ldg(pg);
                     if (pm_update) cq[r] = __ldcg(P.cur_cost + (pg - reinterpret_cast<const unsigned int*>(P.guide)));
                 }
-#endif
                 vi++;
                 pg += P.W;
             }
@@ -1034,9 +899,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
         long long ostride;
         if (P.out_compact) { orow = P.out + (size_t)it.compact_off + t; ostride = it.compact_stride; }
         else { orow = P.out + (size_t)it.oy0 * P.out_pitch + XE; ostride = P.out_pitch; }
-#if LEXP_PDL
         bool prior_grids_done = false;
-#endif
         for (int c = 0; c < nChunks; c++) {
             {
                 LEXP_TRACE_LOAD_WAIT(gq[kCH - 1]);
@@ -1090,16 +953,14 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
                                 }
                                 cpix += (size_t)P.W;
                             } else {
-#if LEXP_PDL
-                            if (!prior_grids_done) {  // write-after-write order against the previous launch of the stream
+                                if (!prior_grids_done) {  // write-after-write order against the previous launch of the stream
 #ifndef LEXP_EMU
-                                asm volatile("griddepcontrol.wait;" ::: "memory");
+                                    asm volatile("griddepcontrol.wait;" ::: "memory");
 #endif
-                                prior_grids_done = true;
-                            }
-#endif
-                            *orow = q;
-                            orow += ostride;
+                                    prior_grids_done = true;
+                                }
+                                *orow = q;
+                                orow += ostride;
                             }
                         }
                     }
@@ -1128,20 +989,6 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) lexp_fused_kernel(const KP
             }
         }
     }
-#if LEXP_TMA_ON
-    else {
-        // =========================================================================== team T (one lane): the statistics ring's producer
-        // chunk k goes to stage k % NS once team C's 96 threads have read chunk k - NS out of it (empty barrier); NS chunks of lead
-        if (lane == 0)
-            for (int k = 0; k < nChunks; k++) {
-                if (k >= LEXP_STATS_STAGES) {
-                    mbar_wait(s_empty + (k % LEXP_STATS_STAGES), (unsigned)(((k / LEXP_STATS_STAGES) - 1) & 1));
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // team C's generic-proxy reads, then the async-proxy refill
-                }
-                tma_issue(k);
-            }
-    }
-#endif
 #if LEXP_TRACE
     if (lane == 0 && P.trace) {
         long long* o = P.trace + ((size_t)blockIdx.x * (kThreads / 32) + warp) * 4;

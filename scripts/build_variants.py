@@ -1,7 +1,6 @@
 #!/usr/bin/env python
-"""Builds the prepared build-time kernel variants of lexp_kernels.cuh next to the product library, as
-variants/liblexp_cuda_<name>.so (git-ignored, but shipped to the GPU box), and prints the ptxas resource lines.
-Run here (nvcc cross-compiles), then `gpurun -- bash scripts/gpu_variants.sh tma4 r1`."""
+"""Builds the diagnosis build of lexp_kernels.cuh (-DLEXP_TRACE=1) next to the product library, as
+variants/liblexp_cuda_trace.so (git-ignored), and prints the ptxas resource lines.  scripts/gpu_trace.sh runs it on the GPU."""
 import os
 import re
 import subprocess
@@ -12,12 +11,6 @@ sys.path.insert(0, ROOT)
 from localexpstereo_b200 import build as B  # noqa: E402
 
 VARIANTS = {
-    "nopdl": ["-DLEXP_PDL=0"],                      # the round-2 defaults switched off one at a time (PDL and ROWTAB are on by default)
-    "norowtab": ["-DLEXP_A_ROWTAB=0"],
-    "r1": ["-DLEXP_PDL=0", "-DLEXP_A_ROWTAB=0"],    # the round-1 kernel
-    "tma3": ["-DLEXP_STATS_TMA=1", "-DLEXP_STATS_STAGES=3"],   # team C's statistics staged by the TMA unit (cp.async.bulk + mbarrier ring)
-    "tma4": ["-DLEXP_STATS_TMA=1", "-DLEXP_STATS_STAGES=4"],
-    "tma5": ["-DLEXP_STATS_TMA=1", "-DLEXP_STATS_STAGES=5"],
     "trace": ["-DLEXP_TRACE=1"],                    # diagnosis: per-team wait / busy cycles of every launch (scripts/gpu_trace.sh)
 }
 

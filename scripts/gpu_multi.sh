@@ -1,4 +1,4 @@
-# gpurun --gpus N -- 'VARIANT=pdl EXTRA="" bash scripts/gpu_multi.sh N'   (VARIANT: a library from scripts/build_variants.py, optional)
+# On a machine with N GPUs: VARIANT=trace EXTRA="" bash scripts/gpu_multi.sh N   (VARIANT: a library from scripts/build_variants.py, optional)
 cd $GRAFT_REPO_ROOT
 N=$1
 mkdir -p gpurun_out

@@ -4,7 +4,7 @@ builds the emulator library with AddressSanitizer -- "device" buffers and the dy
 blocks, so the first byte the kernel reads or writes out of bounds is reported -- and drives the fuzz tests through it.
 
     python tests/emu/asan_fuzz.py [first_seed last_seed]       (re-executes itself with libasan preloaded)
-    LEXP_ASAN_DEFS="-DLEXP_PDL=0 -DLEXP_A_ROWTAB=0" python tests/emu/asan_fuzz.py 0 40      (a build-time kernel variant)
+    LEXP_ASAN_DEFS="-DLEXP_TRACE=1" python tests/emu/asan_fuzz.py 0 40      (the diagnosis build)
 """
 import ctypes as C
 import os

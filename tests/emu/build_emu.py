@@ -13,7 +13,7 @@ SO = os.path.join(HERE, "liblexp_emu.so")
 
 
 def build(force=False, defs=(), tag=""):
-    """`defs`: extra -D flags selecting a build-time kernel variant (e.g. ("-DLEXP_A_ROWTAB=0",)), `tag` names its library."""
+    """`defs`: extra -D flags selecting a build-time kernel variant (e.g. ("-DLEXP_TRACE=1",)), `tag` names its library."""
     so = SO if not tag else os.path.join(HERE, f"liblexp_emu_{tag}.so")
     if os.environ.get("LEXP_EMU_NO_REBUILD") and os.path.exists(so):  # worker processes of a test: the parent has built it
         return so

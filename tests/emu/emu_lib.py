@@ -12,7 +12,7 @@ if HERE not in sys.path:
 
 _emu = {}
 
-VARIANTS = {"": (), "r1": ("-DLEXP_PDL=0", "-DLEXP_A_ROWTAB=0"), "trace": ("-DLEXP_TRACE=1",)}  # build-time kernel variants (lexp_kernels.cuh), "" = the shipped kernel
+VARIANTS = {"": (), "trace": ("-DLEXP_TRACE=1",)}  # build-time kernel variants (lexp_kernels.cuh), "" = the shipped kernel
 
 
 def load(variant=""):

@@ -92,7 +92,7 @@ def test_emu_result_does_not_depend_on_the_thread_schedule(scene):
     assert np.array_equal(outs[0], outs[1]) and np.array_equal(outs[0], outs[2])
 
 
-def test_emu_concurrent_calls_are_combined_into_batched_launches(scene, monkeypatch):
+def test_emu_concurrent_calls_are_combined_into_batched_launches(scene):
     """lexp_eval_cell from many threads at once (the reference's unchanged OpenMP loop): calls that arrive while the device is
     busy must be served together by one launch, with exactly the results of one-call-at-a-time evaluation."""
     import numpy as np
@@ -122,12 +122,10 @@ def test_emu_concurrent_calls_are_combined_into_batched_launches(scene, monkeypa
                 outs.append(list(ex.map(one, range(len(cells)))))
         return outs
 
-    monkeypatch.setenv("LEXP_COMBINE", "0")
     E0 = L.CostVolumeEnergy(imL, imR, volL, volR, prm, D - 1)
-    ref = sweep(E0, 1)
+    ref = sweep(E0, 1)   # one caller at a time: every call takes the plain single-cell path
     assert E0.combine_stats == (0, 0)
     E0.close()
-    monkeypatch.delenv("LEXP_COMBINE")
     E1 = L.CostVolumeEnergy(imL, imR, volL, volR, prm, D - 1)
     got = sweep(E1, 12)
     batches, calls = E1.combine_stats
